@@ -4,6 +4,7 @@
   python bench.py --gpus 1 --steps K --warmup W                 engine arm (this repo, sm_100a kernels)
   torchrun ... bench.py --gpus N ...                              one rank per GPU, weak scaling (fixed images per GPU)
   python bench.py --impl reference ...                            the reference algorithm on the host cores (oracle port)
+  python bench.py ... --dump-outputs DIR                          also write the last timed step's infer() outputs to DIR/*.npy
 
 A "step" is one `MoGeModel.infer()` over one batch of synthetic 518x518 images per GPU.  Rank 0 prints ONE JSON line.
   value  : images/s with the inputs already resident in HBM (device-timed, max over ranks)
@@ -52,7 +53,13 @@ def parse():
                     "~700-token ViT-L-normal bf16 batch (configs[2]); 5: ViT-B resolution / aspect sweep (configs[4])")
     ap.add_argument("--no-gpu-baseline", action="store_true", help="skip the same-box PyTorch-CUDA comparator (gpu_baseline)")
     ap.add_argument("--gpu-baseline-kernels", default=None, help="write the torch.profiler kernel list of one batch-1 comparator pass here")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the infer() outputs of the last timed step (rank 0) to DIR/<name>.npy as float32; above 64 MB in all, "
+                         "a fixed, seeded sample of pixels (see dump_outputs)")
+    a = ap.parse_args()
+    if a.dump_outputs and (a.impl != "engine" or a.config != 0):
+        ap.error("--dump-outputs applies to the engine arm of the default workload")
+    return a
 
 
 def peaks():
@@ -96,6 +103,32 @@ class ClockSampler:
         reasons = sorted({names[i] for r in self.rows if len(r) >= 7 for i in range(4) if r[3 + i].lower().startswith("active")})
         return {"sm_mhz": statistics.median(sm) if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": reasons, "samples": len(self.rows)}
+
+
+DUMP_BYTES = 64 * 10**6
+
+
+def dump_outputs(out, path, H, W):
+    """Write one infer() result to `path`/<name>.npy as float32 (mask as 0 / 1).  Pixels outside the mask, which infer() fills
+    with inf in points / depth and with 0 in normal, are written as 0: every file is finite, and mask.npy tells which pixels
+    hold values.  When the (B, H, W[, C]) maps would exceed DUMP_BYTES in all, every map keeps the same fixed, seeded sample of
+    pixels: maps become (B, n[, C]) and the row-major pixel indices into H x W are written as pixel_index.npy (float64).
+    Same arguments -> same inputs -> comparable files across builds."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    out = {k: v.float().cpu() for k, v in out.items()}
+    maps = {k: v for k, v in out.items() if v.dim() >= 3 and tuple(v.shape[1:3]) == (H, W)}
+    if "mask" in maps:
+        valid = maps["mask"] > 0
+        maps = {k: torch.where(valid if v.dim() == 3 else valid[..., None], v, 0.0) for k, v in maps.items()}
+    rest = sum(v.numel() * 4 for k, v in out.items() if k not in maps) + 128 * (len(out) + 1)       # + .npy headers
+    n = min(H * W, (DUMP_BYTES - rest) // (sum(v.numel() // (H * W) for v in maps.values()) * 4 + 8))
+    if n < H * W:
+        idx = torch.randperm(H * W, generator=torch.Generator().manual_seed(0))[:n].sort().values
+        np.save(os.path.join(path, "pixel_index.npy"), idx.double().numpy())
+        maps = {k: v.flatten(1, 2)[:, idx] for k, v in maps.items()}
+    for k, v in {**out, **maps}.items():
+        np.save(os.path.join(path, k + ".npy"), v.contiguous().numpy())
 
 
 def host_threads():
@@ -290,8 +323,10 @@ def run_engine(a):
         barrier()
         return float(ms.item())
 
+    last_out = [None]
+
     def step_dev():
-        model.infer(dev_in, num_tokens=a.tokens)
+        last_out[0] = model.infer(dev_in, num_tokens=a.tokens)
 
     def step_e2e():
         x = host_in.to(dev, non_blocking=True)
@@ -306,6 +341,9 @@ def run_engine(a):
         sampler.start()
     ms_dev = timed(step_dev, a.steps)
     clocks = sampler.stop() if rank == 0 else None
+    if a.dump_outputs and rank == 0:
+        dump_outputs(last_out[0], a.dump_outputs, R, R)
+    last_out[0] = None
     for _ in range(min(a.warmup, 2)):
         step_e2e()
     ms_e2e_serial = timed(step_e2e, a.steps)

@@ -29,20 +29,30 @@ def test_port_matches_reference_golden(name, golden_dir):
     sd = make_state_dict(cfg, meta["seed"], well_posed=opt.get("well_posed", False))
     B, H, W = meta["shape"]
     img = synthetic_images(B, H, W, meta["seed"])
-    s = meta["stride"]
+    s, si = meta["stride"], meta.get("infer_stride", meta["stride"])
     nt = meta["num_tokens"] or default_num_tokens(cfg["num_tokens_range"])
     fwd = moge_port.forward(cfg, sd, img, nt)
     for k, ref in gold["forward"].items():
         got = fwd[k][:, ::s, ::s] if fwd[k].dim() >= 3 else fwd[k]
         assert rel_l2(got, ref) < 2e-5, k
-    inf = moge_port.infer(cfg, sd, img, num_tokens=meta["num_tokens"])
+    # infer() is forward() followed by postprocess().  On a random-weight (ill-posed) point map the focal/shift solve stops on
+    # SciPy's ftol rule and turns the host-dependent 1e-6 rounding of an fp32 forward() (thread count, vector width) into up to
+    # 3e-3 in the outputs.  So postprocess() is pinned on the reference's own forward() outputs wherever the golden stores them
+    # whole, and well-posed maps are compared end to end as well.
+    runs = []
+    if s == 1:
+        gf = gold["forward"]
+        runs.append(moge_port.postprocess(gf.get("points"), gf.get("normal"), gf.get("mask"), gf.get("metric_scale"), W / H))
+    if s != 1 or opt.get("well_posed", False):
+        runs.append(moge_port.infer(cfg, sd, img, num_tokens=meta["num_tokens"]))
     m = gold["infer"]["mask"]
-    assert (inf["mask"][:, ::s, ::s] == m).float().mean() > 0.9999
-    for k in ("points", "depth", "normal"):
-        if k in gold["infer"]:
-            got = inf[k][:, ::s, ::s]
-            assert rel_l2(got[m], gold["infer"][k][m]) < 1e-4, k
-    assert rel_l2(inf["intrinsics"], gold["infer"]["intrinsics"]) < 1e-5
+    for inf in runs:
+        assert (inf["mask"][:, ::si, ::si] == m).float().mean() > 0.9999
+        for k in ("points", "depth", "normal"):
+            if k in gold["infer"]:
+                got = inf[k][:, ::si, ::si]
+                assert rel_l2(got[m], gold["infer"][k][m]) < 1e-4, k
+        assert rel_l2(inf["intrinsics"], gold["infer"]["intrinsics"]) < 1e-5
 
 
 def test_port_focal_shift_golden(golden_dir):
